@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — RGB-D frames/s of the PlanarSLAM per-frame hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one pass of the hot path over 7104 frames of a 256-frame synthetic 640x480 RGB-D sequence ("room corner", planarslam_b200/synth.py): four library
@@ -107,6 +107,36 @@ def _peaks():
         return float(p["hbm_gbs"]), "measured"
     except Exception:
         return 6650.0, "fallback"
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def save_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32 (float32, and integers all below 2^24 in magnitude) or float64 (everything else), so every value
+    stays exact; structured records become one column per scalar field.  Every written value is finite: where an output holds NaN or infinity (the
+    direction of a rejected 3-D line, the normal of a pixel without depth), the value is written as 0 and out_dir/<name>_nonfinite.npy (float32, same
+    shape) records 1 for NaN, 2 for +inf, 3 for -inf and 0 elsewhere.  Fails if the files would exceed DUMP_LIMIT bytes in all."""
+    from numpy.lib import recfunctions
+    conv = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype.names:
+            a = recfunctions.structured_to_unstructured(a, dtype=np.float64)
+        small_int = a.dtype.kind in "iub" and (a.size == 0 or int(np.abs(a.astype(np.int64)).max()) < (1 << 24))
+        a = a.astype(np.float32 if a.dtype == np.float32 or small_int else np.float64)
+        bad = ~np.isfinite(a)
+        if bad.any():
+            conv[name + "_nonfinite"] = np.select([np.isnan(a), a == np.inf, a == -np.inf], [1, 2, 3], 0).astype(np.float32)
+            a = np.where(bad, 0, a).astype(a.dtype)
+        conv[name] = a
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
 
 
 def make_frames(n_distinct=DISTINCT_FRAMES, world=1):
@@ -442,8 +472,14 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (a fixed sample of frames; rank 0)")
     ap.add_argument("--cpu-worker", default=None, help=argparse.SUPPRESS)       # internal: child process of the CPU arm
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     if args.cpu_worker:
         cpu_worker_main(json.loads(args.cpu_worker))
         return
@@ -719,6 +755,81 @@ def main():
             dist.barrier()
         torch.cuda.synchronize(dev)
 
+    def dump_last_step():
+        """What the last timed step left in the stage buffers: ORB, PEAC and pose hold the step's last sub-batch, LSD every frame of the step.  A fixed
+        sample of frames (seed 0) keeps the files small; entries past a frame's count are zeroed, since the buffers are reused without clearing."""
+        torch.cuda.synchronize(dev)
+        rng = np.random.default_rng(0)
+        sb = np.sort(rng.choice(SUB_BATCH, min(8 // AREA, SUB_BATCH), replace=False))            # frames of the last sub-batch (image-sized outputs)
+        fs = np.sort(rng.choice(FRAMES_PER_STEP, min(64, FRAMES_PER_STEP), replace=False))        # frames of the step (LSD)
+        last = (SUBS_PER_STEP - 1) * SUB_BATCH
+        host = lambda t, rows: t[torch.as_tensor(rows, device=dev)].cpu().numpy()
+
+        def upto(a, n):
+            a = a.copy()
+            for i, k in enumerate(n):
+                a[i, int(k):] = 0
+            return a
+        out = {}
+        if "orb" in STAGES:
+            n_all = d_n.cpu().numpy()
+            n = n_all[last + sb]
+            out["orb_n"] = n_all[last:last + SUB_BATCH]
+            out["orb_keypoints"] = upto(host(d_kps, sb).view(KEYPOINT_DTYPE)[..., 0], n)
+            out["orb_descriptors"] = upto(host(d_desc, sb), n)
+            if EXTRAS:
+                out["stereo_u_right"], out["stereo_depth"] = upto(host(d_ur, sb), n), upto(host(d_dz, sb), n)
+                q = sb[sb < SUB_BATCH - 1]                                   # MatchORBPoints: frame q + 1 against frame q
+                out["match_knn_idx"] = upto(host(d_midx, q), n_all[last + q + 1])
+                out["match_knn_dist"] = upto(host(d_mdist, q), n_all[last + q + 1])
+                ngood = d_ngood.cpu().numpy()[:SUB_BATCH - 1]
+                out["match_n_good"] = ngood
+                out["match_good"] = upto(host(d_good, q), ngood[q])               # the gated MatchORBPoints result
+                if xch is not None:                                               # key-frame exchange of the step's first sub-batch, every key frame
+                    kf = np.minimum(np.arange(KF) * kf_stride, SUB_BATCH - 1)
+                    out["exchange_idx"] = upto(d_xidx.cpu().numpy(), n_all[kf])
+                    out["exchange_dist"] = upto(d_xdist.cpu().numpy(), n_all[kf])
+        if "peac" in STAGES:
+            npl_all = d_npl.cpu().numpy()
+            npl = npl_all[last + sb]
+            moff = upto(host(d_moff, sb), npl + 1)
+            out["peac_n_planes"] = npl_all[last:last + SUB_BATCH]
+            out["peac_planes"] = upto(host(d_planes, sb).view(PLANE_DTYPE)[..., 0], npl)
+            out["peac_labels"] = host(d_labels, sb)
+            out["peac_member_offsets"] = moff
+            out["peac_members"] = upto(host(d_members, sb), moff[np.arange(len(sb)), npl])
+            if EXTRAS:
+                pn = host(d_pp_n, sb)
+                poff = upto(host(d_pp_off, sb), pn + 1)
+                out["planes_n"], out["planes_src"], out["planes_coef"] = pn, upto(host(d_pp_src, sb), pn), upto(host(d_pp_coef, sb), pn)
+                out["planes_point_offsets"], out["planes_points"] = poff, upto(host(d_pp_pts, sb), poff[np.arange(len(sb)), pn])
+                out["planes_status"] = d_pp_status.cpu().numpy()
+                out["surface_normals"] = host(d_sn3, sb)
+                out["surface_normal_records"] = host(d_sn8, sb)                   # normal, cameraPosition, FramePosition
+                out["manhattan"] = host(d_mres, sb).view(MANHATTAN_RESULT_DTYPE)[..., 0]
+                out["manhattan_normal_mask"], out["manhattan_direction_mask"] = host(d_nmask, sb), host(d_dmask, sb)
+        if "lsd" in STAGES:
+            nkl = d_nkl.cpu().numpy()[fs]
+            out["lsd_n_lines"] = d_nkl.cpu().numpy()
+            out["lsd_keylines"] = upto(host(d_kl, fs).view(KEYLINE_DTYPE)[..., 0], nkl)
+            out["lsd_line_functions"] = upto(host(d_lf, fs), nkl)
+            if EXTRAS:
+                out["lsd_descriptors"] = upto(host(d_ldesc, fs), nkl)
+                l3 = upto(host(d_l3d, fs).view(LINE3D_DTYPE)[..., 0], nkl)
+                out["lines3d"] = l3[[f for f in LINE3D_DTYPE.names if f != "inliers"]]
+                out["lines3d_inliers_u32"] = np.ascontiguousarray(l3["inliers"]).view(np.uint32).reshape(l3.shape + (2,))       # a 64-bit mask: two exact halves
+                out["lines3d_draws"] = d_drawn.cpu().numpy()
+        if "pose" in STAGES:
+            res = opt.fetch()
+            out["pose_Tcw"] = np.stack([r["Tcw_d"] for r in res])
+            out["pose_Tcw_float"] = np.stack([r["Tcw"] for r in res])
+            out["pose_n_inliers"] = np.array([r["n_inliers"] for r in res], np.int32)
+            out["pose_trace_i"], out["pose_trace_d"] = np.stack([r["trace_i"] for r in res]), np.stack([r["trace_d"] for r in res])
+            for k in ("outlier_pt", "outlier_line", "outlier_plane", "outlier_par", "outlier_ver"):
+                out["pose_" + k] = np.concatenate([res[i][k] for i in sb])
+        total = save_outputs(args.dump_outputs, out)
+        print(f"bench: {len(out)} outputs of the last timed step ({total} bytes) written to {args.dump_outputs}", file=sys.stderr)
+
     # ---- device-resident throughput ----
     steps_dev(max(args.warmup, 3))
     barrier()
@@ -740,6 +851,10 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = world * FRAMES_PER_STEP * args.steps / (ms_max / 1e3)
+    if args.dump_outputs:
+        if rank == 0:
+            dump_last_step()
+        barrier()                  # the other ranks' next exchange waits on rank 0's epoch flag: keep them from starting it during the dump
 
     # ---- per-kernel roofline pass (event-bracketed launches, same workload, outside the timed regions) ----
     # one stage family at a time, so a launch's duration is not inflated by kernels of the other two streams

@@ -1,6 +1,11 @@
 """ctypes access to oracle/_ref/*.so - the REFERENCE's own sources compiled in the build container (make -C oracle ref) against the
 stand-in headers of oracle/ref/shims/.  Test infrastructure only; the libraries are prebuilt artefacts on the GPU box."""
+import atexit
 import ctypes as C
+import functools
+import hashlib
+import inspect
+import json
 import os
 import subprocess
 
@@ -16,6 +21,161 @@ def _load(name):
     if not os.path.exists(path) and os.path.isdir("/root/reference/src"):
         subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True, stdout=subprocess.DEVNULL)
     return C.CDLL(path) if os.path.exists(path) else None
+
+
+# Recorded answers.  The compiled reference exists only where the reference's sources were, so every ref_* call below that a test makes
+# is answered, where its library is absent, from the outputs the library gave for the same arguments: tests/golden/reference_calls/<function>.npz,
+# keyed by a SHA-1 of the arguments.  Running the tests with PSLAM_REF_RECORD=<dir> where the libraries are built writes <dir>/<function>.npz.
+# A call with no recorded answer is an error, never a skip.  Outputs larger than DIGEST_OVER bytes of the functions recorded with digest=True
+# (label maps, key points, descriptors, 3-D lines: only ever compared for equality) are kept as their SHA-1; compare them with same().
+CALLS_DIR = os.path.join(ROOT, "tests", "golden", "reference_calls")
+DIGEST_OVER = 256
+_recording = {}
+
+
+class Digest:
+    """A recorded output array kept as its dtype, shape and SHA-1 of its bytes."""
+
+    def __init__(self, descr, shape, sha1):
+        self.descr, self.shape, self.sha1 = descr, tuple(shape), sha1
+
+    def __len__(self):
+        return self.shape[0]
+
+    def matches(self, a) -> bool:
+        a = np.ascontiguousarray(a)
+        return str(a.dtype.descr) == self.descr and a.shape == self.shape and _sha1(a) == self.sha1
+
+
+def _sha1(a):
+    """SHA-1 of the values of a: every NaN and both zeros hash alike, as np.array_equal(equal_nan=True) compares them."""
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a + 0.0).astype(a.dtype)
+    return hashlib.sha1(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def same(a, b) -> bool:
+    """a equals b, either of which may be a reference output kept as a Digest (NaNs compare equal, as in a Digest)."""
+    if isinstance(b, Digest):
+        a, b = b, a
+    if isinstance(a, Digest):
+        return a.matches(b)
+    a, b = np.ascontiguousarray(a), np.ascontiguousarray(b)
+    if a.dtype.kind == "V" or b.dtype.kind == "V":             # records (key points): byte for byte, as a Digest hashes them
+        return a.dtype.itemsize == b.dtype.itemsize and a.shape == b.shape and a.tobytes() == b.tobytes()
+    return np.array_equal(a, b, equal_nan=a.dtype.kind == "f" and b.dtype.kind == "f")
+
+
+def _feed(h, x):
+    if isinstance(x, (np.ndarray, np.generic)):
+        a = np.ascontiguousarray(x)
+        h.update(f"a{a.dtype.descr}{a.shape}".encode())
+        h.update(a.tobytes())
+    elif isinstance(x, dict):
+        h.update(b"d%d" % len(x))
+        for k in sorted(x):
+            _feed(h, k)
+            _feed(h, x[k])
+    elif isinstance(x, (list, tuple)):
+        h.update(b"l%d" % len(x))
+        for v in x:
+            _feed(h, v)
+    elif isinstance(x, RefVocabulary):
+        _feed(h, x.text)
+    else:
+        h.update(f"{type(x).__name__}:{x!r}".encode())
+
+
+def _flatten(x, arrays, digest, whole=(), omit=()):
+    """JSON description of x whose arrays are appended to arrays.  whole: top-level keys / indices never digested; omit: top-level keys not stored."""
+    if isinstance(x, np.ndarray):
+        if digest and x.nbytes > DIGEST_OVER:
+            a = np.ascontiguousarray(x)
+            return {"digest": [str(a.dtype.descr), list(a.shape), _sha1(a)]}
+        arrays.append(x)
+        return {"a": len(arrays) - 1}
+    if isinstance(x, np.generic):
+        arrays.append(np.asarray(x))
+        return {"s": len(arrays) - 1}
+    if isinstance(x, dict):
+        return {"d": [[k, _flatten(v, arrays, digest and k not in whole, whole=())] for k, v in x.items() if k not in omit]}
+    if isinstance(x, (list, tuple)):
+        return {"t" if isinstance(x, tuple) else "l": [_flatten(v, arrays, digest and i not in whole, whole=()) for i, v in enumerate(x)]}
+    assert x is None or isinstance(x, (bool, int, float, str)), type(x)
+    return {"v": x}
+
+
+def _unflatten(spec, arrays):
+    (kind, v), = spec.items()
+    if kind == "a":
+        return arrays[v].copy()
+    if kind == "s":
+        return arrays[v][()]
+    if kind == "digest":
+        return Digest(*v)
+    if kind == "d":
+        return {k: _unflatten(s, arrays) for k, s in v}
+    if kind in ("t", "l"):
+        items = [_unflatten(s, arrays) for s in v]
+        return tuple(items) if kind == "t" else items
+    return v
+
+
+def _write_recording():
+    out_dir = os.environ["PSLAM_REF_RECORD"]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, calls in _recording.items():
+        path = os.path.join(out_dir, name + ".npz")
+        entries = dict(np.load(path)) if os.path.exists(path) else {}
+        for key, (spec, arrays) in calls.items():
+            entries[key + ".spec"] = np.array(json.dumps({"n": len(arrays), "out": spec}))
+            for i, a in enumerate(arrays):
+                entries[f"{key}.{i}"] = a
+        np.savez_compressed(path, **entries)
+
+
+_replay = {}
+LBA_FLOAT_COPIES = ("kf_Tcw", "pt_Xw", "line_Xw", "plane_Xw")      # the float write-back next to the *_d doubles the tests compare
+
+
+def _recorded(lib_getter, digest=False, whole=lambda args: (), omit=()):
+    """Decorator of a ref_* function: live where lib_getter() finds the library (and recorded if PSLAM_REF_RECORD is set), replayed otherwise.
+    Calls with impl != "ref" (the product's adapter) are never recorded.  whole(arguments): top-level outputs of that call stored whole even with
+    digest=True; omit: keys of a dict result that no test reads, left out of the recording."""
+    def wrap(fn):
+        sig = inspect.signature(fn)
+
+        @functools.wraps(fn)
+        def call(*args, **kw):
+            bound = sig.bind(*args, **kw)
+            bound.apply_defaults()
+            if bound.arguments.get("impl", "ref") != "ref":
+                return fn(*args, **kw)
+            live = lib_getter() is not None
+            if live and not os.environ.get("PSLAM_REF_RECORD"):
+                return fn(*args, **kw)
+            h = hashlib.sha1(fn.__qualname__.encode())
+            _feed(h, {k: v for k, v in bound.arguments.items() if k != "impl"})
+            key = h.hexdigest()
+            if live:
+                out = fn(*args, **kw)
+                if not _recording:
+                    atexit.register(_write_recording)
+                arrays = []
+                spec = _flatten(out, arrays, digest, whole(bound.arguments), omit)
+                _recording.setdefault(fn.__qualname__, {})[key] = (spec, arrays)
+                return out
+            if fn.__qualname__ not in _replay:
+                path = os.path.join(CALLS_DIR, fn.__qualname__ + ".npz")
+                _replay[fn.__qualname__] = np.load(path) if os.path.exists(path) else {}
+            rec = _replay[fn.__qualname__]
+            if key + ".spec" not in rec:
+                raise LookupError(f"no recorded answer of the compiled reference for this call of {fn.__qualname__} (key {key}): record it with "
+                                  "PSLAM_REF_RECORD=<dir> where oracle/_ref is built and add <dir>/*.npz to tests/golden/reference_calls/")
+            spec = json.loads(str(rec[key + ".spec"]))
+            return _unflatten(spec["out"], [rec[f"{key}.{i}"] for i in range(spec["n"])])
+        return call
+    return wrap
 
 
 _peac = None
@@ -39,6 +199,7 @@ def peac_lib():
     return _peac
 
 
+@_recorded(peac_lib, digest=True)
 def ref_peac_run(depth16, K=(535.4, 539.2, 320.1, 247.6), scale=np.float32(1.0 / 5000.0)):
     """PlaneDetection::readDepthImage + runPlaneDetection of the reference itself.  Returns (labels int32 [h][w] = membershipImg,
     planes [(normal3 + center3 + mse + curvature, N)], plane_vertices_ lists)."""
@@ -85,6 +246,7 @@ def orb_lib():
     return _orb
 
 
+@_recorded(orb_lib, digest=True, whole=lambda a: () if a["monotonic_alloc"] else (0,))
 def ref_orb_extract(gray, nfeatures=1000, scale=1.2, nlevels=8, ini_th=20, min_th=7, monotonic_alloc=True, cap=8192):
     """Planar_SLAM::ORBextractor::operator() of the reference itself. Returns (key points as 28-byte records, descriptors [n][32]).
     monotonic_alloc: the library's allocations come from a bump arena, so the quadtree's address ties follow creation order."""
@@ -139,13 +301,18 @@ class RefVocabulary:
     """ORBVocabulary of the reference (DBoW2 compiled from /root/reference) loaded from a text file."""
 
     def __init__(self, path: str):
+        with open(path) as f:
+            self.text = f.read()                   # what identifies the vocabulary in a recorded call
         self.L = bow_lib()
-        self.h = C.c_void_p(self.L.ref_voc_load(path.encode()))
-        assert self.h.value, "loadFromTextFile failed"
+        if self.L is not None:
+            self.h = C.c_void_p(self.L.ref_voc_load(path.encode()))
+            assert self.h.value, "loadFromTextFile failed"
 
+    @_recorded(bow_lib)
     def size(self):
         return self.L.ref_voc_size(self.h)
 
+    @_recorded(bow_lib, digest=True)
     def transform(self, features: np.ndarray, levelsup: int = 4):
         f = np.ascontiguousarray(features, np.uint8)
         n = len(f)
@@ -157,6 +324,7 @@ class RefVocabulary:
         return dict(word_id=o["word_id"][:nw], word_val=o["word_val"][:nw], node_id=o["node_id"][:nn], node_off=o["node_off"][:nn + 1],
                     node_feat=o["node_feat"][:o["node_off"][nn]])
 
+    @_recorded(bow_lib)
     def score(self, a: dict, b: dict) -> float:
         ia, va = np.ascontiguousarray(a["word_id"], np.int32), np.ascontiguousarray(a["word_val"], np.float64)
         ib, vb = np.ascontiguousarray(b["word_id"], np.int32), np.ascontiguousarray(b["word_val"], np.float64)
@@ -183,6 +351,7 @@ def line3d_lib():
     return _line3d
 
 
+@_recorded(line3d_lib, digest=True)
 def ref_lines3d_frame(keylines, depth, cam, seed=1, skip=0):
     """The reference's compPt3dCov + extract3dline_mahdist (src/LineExtractor.cpp, libc rand() after srand(seed) and `skip` draws) inside a
     restated Frame::isLineGood loop.  Same outputs as oracle_lib.lines3d_frame (without the draw count)."""
@@ -214,6 +383,7 @@ def pose_lib():
     return _pose
 
 
+@_recorded(pose_lib)
 def ref_pose_optimization(p: dict):
     """PoseOptimization run by the reference's own g2o, edges and Converter (compiled against the Eigen stand-in) on a planarslam_b200.synth_pose problem;
     the graph construction and the four optimise-and-classify rounds are restated in oracle/ref/pose_driver.cc.  Same keys as oracle_lib.pose_optimization."""
@@ -229,6 +399,7 @@ def ref_pose_optimization(p: dict):
                 outlier_ver=o[4][:s.n_ver], iterations=it)
 
 
+@_recorded(pose_lib)
 def ref_translation_optimization(p: dict):
     """TranslationOptimization by the reference's g2o and OnlyTranslation edges (oracle/ref/pose_driver.cc)."""
     import oracle_lib
@@ -242,6 +413,7 @@ def ref_translation_optimization(p: dict):
     return dict(Tcw_d=Td, n_inliers=n, outlier_pt=o[0][:s.n_points], outlier_line=o[1][:s.n_lines], outlier_plane=o[2][:s.n_planes], iterations=it)
 
 
+@_recorded(pose_lib, omit=LBA_FLOAT_COPIES)
 def ref_local_bundle_adjustment(p: dict) -> dict:
     """LocalBundleAdjustment run by the reference's own g2o (BlockSolver_6_3 + Schur complement + Levenberg-Marquardt), edges and vertices on a
     planarslam_b200.synth_lba problem; the graph construction, the 5 + 10 iterations with the chi-square gating in between and the erase lists are
@@ -287,6 +459,7 @@ def _impl(impl):
     return (match_lib(), "ref_") if impl == "ref" else (adapter_lib(), "adp_")
 
 
+@_recorded(match_lib, digest=True, whole=lambda a: (1,))
 def ref_search_by_projection_map(fv: dict, m: dict, th: float, nnratio: float, matches0: np.ndarray, impl: str = "ref"):
     """Tracking::SearchLocalPoints' frustum loop + ORBmatcher::SearchByProjection(Frame&, vector<MapPoint*>&, th) by the reference's own code
     (impl="adp": by the product's adapter class of the same signature, on the same objects).  Same arguments and returns as oracle_lib.search_by_projection_map."""
@@ -301,6 +474,7 @@ def ref_search_by_projection_map(fv: dict, m: dict, th: float, nnratio: float, m
     return n, matches, in_view[:m["n"]]
 
 
+@_recorded(match_lib)
 def ref_search_by_projection_last(fv: dict, lf: dict, m: dict, th: float, mono: bool, check_ori: bool, matches0: np.ndarray, impl: str = "ref"):
     """ORBmatcher::SearchByProjection(Frame& CurrentFrame, const Frame& LastFrame, th, bMono) by the reference's own code (impl="adp": the product's adapter)."""
     import oracle_lib
@@ -313,6 +487,7 @@ def ref_search_by_projection_last(fv: dict, lf: dict, m: dict, th: float, mono: 
     return n, matches
 
 
+@_recorded(match_lib, digest=True)
 def ref_search_by_bow(kf: dict, frame: dict, nnratio: float = 0.7, check_orientation: bool = True, impl: str = "ref"):
     """ORBmatcher::SearchByBoW(KeyFrame*, Frame&, vector<MapPoint*>&) by the reference's own code (impl="adp": the product's adapter).  Same layout as
     oracle_lib.search_by_bow."""
@@ -331,6 +506,7 @@ def ref_search_by_bow(kf: dict, frame: dict, nnratio: float = 0.7, check_orienta
     return n, match[:nf]
 
 
+@_recorded(match_lib)
 def ref_lines_in_frustum(frame: dict, pos, normal, max_distance, min_distance, cos_limit: float = 0.5):
     """Frame::isInFrustum(MapLine*, cosLimit) by the reference's own code.  Same arguments / returns as oracle_lib.lines_in_frustum."""
     L = match_lib()
@@ -347,6 +523,7 @@ def ref_lines_in_frustum(frame: dict, pos, normal, max_distance, min_distance, c
     return o
 
 
+@_recorded(match_lib, digest=True)
 def ref_line_search_by_projection(frame: dict, map_lines: dict, th: float, nnratio: float, impl: str = "ref"):
     """LSDmatcher::SearchByProjection(Frame&, vector<MapLine*>&, th) by the reference's own code (impl="adp": the product's adapter).  Same layout as
     oracle_lib.line_search_by_projection."""
@@ -364,6 +541,7 @@ def ref_line_search_by_projection(frame: dict, map_lines: dict, th: float, nnrat
     return n, assigned[:nf]
 
 
+@_recorded(match_lib, digest=True)
 def ref_plane_match(T, fc, mc, bad, off, pts, dTh, aTh, verTh, parTh, impl: str = "ref"):
     """PlaneMatcher::SearchMapByCoefficients by the reference's own code (impl="adp": the product's adapter).  Returns (nmatches, match, vertical, parallel)."""
     lib, pre = _impl(impl)
@@ -377,6 +555,7 @@ def ref_plane_match(T, fc, mc, bad, off, pts, dTh, aTh, verTh, parTh, impl: str 
     return n, om[:len(fc)], ov[:len(fc)], op[:len(fc)]
 
 
+@_recorded(match_lib)
 def ref_full_pose_optimization(p: dict, translation_only: bool = False, impl: str = "ref"):
     """Optimizer::PoseOptimization(Frame*) / TranslationOptimization(Frame*) THEMSELVES (src/Optimizer.cc compiled unmodified into libmatch_ref.so) on a
     Frame built from a planarslam_b200.synth_pose problem.  Returns dict(Tcw float32 4x4 - the reference writes the pose back as float -, n_inliers, outlier_*)."""
@@ -393,6 +572,7 @@ def ref_full_pose_optimization(p: dict, translation_only: bool = False, impl: st
                 outlier_par=o[3][:s.n_par], outlier_ver=o[4][:s.n_ver])
 
 
+@_recorded(match_lib, omit=LBA_FLOAT_COPIES)
 def ref_full_local_bundle_adjustment(p: dict, impl: str = "ref") -> dict:
     """Optimizer::LocalBundleAdjustment(KeyFrame*, bool*, Map*) ITSELF (src/Optimizer.cc compiled unmodified into libmatch_ref.so) on a key-frame / landmark graph
     built from a planarslam_b200.synth_lba problem.  Keys of oracle_lib.local_bundle_adjustment (positions as the reference wrote them back: float) plus
@@ -411,6 +591,7 @@ def ref_full_local_bundle_adjustment(p: dict, impl: str = "ref") -> dict:
     return out
 
 
+@_recorded(match_lib, digest=True)
 def ref_full_compute_stereo_from_rgbd(keys_xy, keys_un_xy, depth, bf: float):
     """Frame::ComputeStereoFromRGBD itself (compiled src/Frame.cc).  Same arguments / returns as oracle_lib.compute_stereo_from_rgbd."""
     L = match_lib()
@@ -422,6 +603,7 @@ def ref_full_compute_stereo_from_rgbd(keys_xy, keys_un_xy, depth, bf: float):
     return ur, dz
 
 
+@_recorded(match_lib, digest=True)
 def ref_full_lines3d_frame(keylines, depth, cam, seed=1, skip=0):
     """Frame::isLineGood itself (compiled src/Frame.cc + src/LineExtractor.cpp, libc rand() after srand(seed) and `skip` draws): (mvDepthLine, mvLines3D)."""
     from oracle_lib import KEYLINE_DTYPE
@@ -445,6 +627,7 @@ def track_lib():
     return _track
 
 
+@_recorded(track_lib)
 def ref_track_manhattan_frame(R_last, normals, dirs):
     """Tracking::TrackManhattanFrame itself.  Returns the 3x3 float32 rotation it returns."""
     L = track_lib()
@@ -457,6 +640,7 @@ def ref_track_manhattan_frame(R_last, normals, dirs):
     return out
 
 
+@_recorded(match_lib, digest=True)
 def ref_detect_loop_candidates(db: dict, min_score: float, sentinel: float = -1.0, impl: str = "ref"):
     """KeyFrameDatabase::DetectLoopCandidates by the reference's own code (src/KeyFrameDatabase.cc + DBoW2 L1 scoring).  Same layout as oracle_lib.detect_loop_candidates."""
     lib, pre = _impl(impl)
@@ -471,6 +655,7 @@ def ref_detect_loop_candidates(db: dict, min_score: float, sentinel: float = -1.
     return cand[:n].copy(), words[:n_kf], score[:n_kf]
 
 
+@_recorded(match_lib, digest=True)
 def ref_detect_relocalization_candidates(db: dict, reloc_score: np.ndarray, impl: str = "ref"):
     lib, pre = _impl(impl)
     fn = getattr(lib, pre + "detect_relocalization_candidates")
@@ -483,6 +668,7 @@ def ref_detect_relocalization_candidates(db: dict, reloc_score: np.ndarray, impl
     return cand[:n].copy(), words[:n_kf], score
 
 
+@_recorded(match_lib, digest=True)
 def ref_search_by_bow_kf(kf1: dict, kf2: dict, nnratio: float = 0.75, check_orientation: bool = True, impl: str = "ref"):
     """ORBmatcher::SearchByBoW(KeyFrame*, KeyFrame*, vector<MapPoint*>&) by the reference's own code (impl="adp": the product's adapter)."""
     import oracle_lib
@@ -490,6 +676,7 @@ def ref_search_by_bow_kf(kf1: dict, kf2: dict, nnratio: float = 0.75, check_orie
     return oracle_lib._bow_kf_call(getattr(lib, pre + "search_by_bow_kf"), kf1, kf2, nnratio, check_orientation)
 
 
+@_recorded(match_lib)
 def ref_line_search_by_descriptor(kf_desc, kf_has_ml, f_desc, impl: str = "ref"):
     """LSDmatcher::SearchByDescriptor(KeyFrame*, Frame&, vector<MapLine*>&) by the reference's own code (impl="adp": the product's adapter).  Returns (nmatches,
     match [n_f]: key line of the key frame whose map line the call stores into vpMapLineMatches[j], -1 NULL)."""

@@ -6,7 +6,6 @@ ulp: the oracle does the closing SVD in float, the stand-in of cv::SVD in double
 import os
 
 import numpy as np
-import pytest
 
 import oracle_lib
 import ref_lib
@@ -26,7 +25,6 @@ def test_manhattan_oracle_matches_reference_golden():
         assert np.abs(o["R"] - g[f"R{i}"]).max() < 4e-7, kw
 
 
-@pytest.mark.skipif(ref_lib.track_lib() is None, reason="oracle/_ref/libtrack_ref.so not built and no /root/reference to build it from")
 def test_manhattan_oracle_agrees_with_track_manhattan_frame_itself():
     n_svd = n_plain = 0
     for kw in CASES:

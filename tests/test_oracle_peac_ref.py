@@ -3,13 +3,12 @@
   * live: src/PlaneExtractor.cpp + include/peac/*.hpp compiled unmodified from /root/reference (oracle/_ref/libpeac_ref.so, built by
     `make -C oracle ref` against the container stand-ins of oracle/ref/shims/ - cv::Mat as a typed buffer, and the 3x3 eigen-solver,
     which is the oracle's Jacobi because Eigen is not in this image).  Label image incl. the raw trail counters, plane parameters,
-    supports and member lists must be IDENTICAL.  Skipped where neither the prebuilt library nor /root/reference exists.
+    supports and member lists must be IDENTICAL.  Where the library is absent, its recorded answers (ref_lib) stand in.
   * golden: the same outputs committed as tests/golden/peac_reference.npz (tools/make_golden_ref.py), checked everywhere."""
 import os
 import sys
 
 import numpy as np
-import pytest
 
 import oracle_lib
 import ref_lib
@@ -33,7 +32,6 @@ def test_oracle_peac_matches_reference_golden():
         assert np.array_equal(np.stack([digest(m) for m in o.membership]), g[key + "_members_sha1"]), key
 
 
-@pytest.mark.skipif(ref_lib.peac_lib() is None, reason="oracle/_ref/libpeac_ref.so not built and no /root/reference to build it from")
 def test_oracle_peac_identical_to_compiled_reference():
     scenes = [synth.render_frame(seed=s, frame=3 * s)[1] for s in range(4)]
     scenes += [synth.piecewise_planar_depth(s, n_rect=6 + s, curved=(s % 2 == 0)) for s in range(12)]
@@ -44,7 +42,7 @@ def test_oracle_peac_identical_to_compiled_reference():
     for k, d16 in enumerate(scenes):
         labels, planes, members = ref_lib.ref_peac_run(d16)
         o = oracle_lib.PeacOracle(d16)
-        assert np.array_equal(labels, o.labels), k
+        assert ref_lib.same(labels, o.labels), k
         assert len(planes) == len(o.planes), k
         for i, (d8, N) in enumerate(planes):
             if k == len(scenes) - 1:
@@ -53,19 +51,18 @@ def test_oracle_peac_identical_to_compiled_reference():
                 assert np.allclose(d8, o.planes[i][0], rtol=0, atol=1e-12) and N == o.planes[i][1][0], (k, i)
             else:
                 assert np.array_equal(d8, o.planes[i][0]) and N == o.planes[i][1][0], (k, i)
-            assert np.array_equal(members[i], o.membership[i]), (k, i)
+            assert ref_lib.same(members[i], o.membership[i]), (k, i)
         n_planes += len(planes)
     assert n_planes > 150
 
 
-@pytest.mark.skipif(ref_lib.peac_lib() is None, reason="oracle/_ref/libpeac_ref.so not built and no /root/reference to build it from")
 def test_oracle_peac_identical_to_compiled_reference_other_cameras_and_sizes():
     def same(d16, K, sc):
         labels, planes, members = ref_lib.ref_peac_run(d16, K, sc)
         o = oracle_lib.PeacOracle(d16, K, sc)
-        assert np.array_equal(labels, o.labels) and len(planes) == len(o.planes)
+        assert ref_lib.same(labels, o.labels) and len(planes) == len(o.planes)
         for i, (d8, N) in enumerate(planes):
-            assert np.array_equal(d8, o.planes[i][0]) and N == o.planes[i][1][0] and np.array_equal(members[i], o.membership[i])
+            assert np.array_equal(d8, o.planes[i][0]) and N == o.planes[i][1][0] and ref_lib.same(members[i], o.membership[i])
         return len(planes)
     tum, s5k = (535.4, 539.2, 320.1, 247.6), np.float32(1.0 / 5000.0)
     d = synth.render_frame(seed=3, frame=9)[1]
@@ -76,7 +73,6 @@ def test_oracle_peac_identical_to_compiled_reference_other_cameras_and_sizes():
     assert same(synth.piecewise_planar_depth(3)[:475, :633].copy(), tum, s5k) >= 5                # size not a multiple of the 10 x 10 block
 
 
-@pytest.mark.skipif(ref_lib.peac_lib() is None, reason="oracle/_ref/libpeac_ref.so not built and no /root/reference to build it from")
 def test_oracle_peac_fuzz_vs_compiled_reference():
     """Random image sizes (not multiples of the block size), cameras (some with fy < 0), patch counts, noise levels and hole fractions."""
     rng = np.random.default_rng(5)
@@ -88,8 +84,8 @@ def test_oracle_peac_fuzz_vs_compiled_reference():
         K = (float(rng.uniform(300, 700)), float(rng.uniform(300, 700)) * (1 if it % 5 else -1), w / 2 + float(rng.normal(0, 5)), h / 2 + float(rng.normal(0, 5)))
         labels, planes, members = ref_lib.ref_peac_run(d, K)
         o = oracle_lib.PeacOracle(d, K)
-        assert np.array_equal(labels, o.labels) and len(planes) == len(o.planes), (it, w, h)
+        assert ref_lib.same(labels, o.labels) and len(planes) == len(o.planes), (it, w, h)
         for i, (d8, N) in enumerate(planes):
-            assert np.array_equal(d8, o.planes[i][0]) and N == o.planes[i][1][0] and np.array_equal(members[i], o.membership[i]), (it, i)
+            assert np.array_equal(d8, o.planes[i][0]) and N == o.planes[i][1][0] and ref_lib.same(members[i], o.membership[i]), (it, i)
         n_planes += len(planes)
     assert n_planes > 80

@@ -9,7 +9,6 @@ oracle/ref/pose_driver.cc.  Bar: identical inlier counts and outlier flags of ev
 import os
 
 import numpy as np
-import pytest
 
 import oracle_lib
 import ref_lib
@@ -35,7 +34,6 @@ def test_oracle_pose_matches_reference_golden():
         _same(o, dict(Tcw_d=g[f"c{i}_Tcw_d"], n_inliers=int(g[f"c{i}_n"][0]), **{k: g[f"c{i}_{k}"] for k in FLAGS}))
 
 
-@pytest.mark.skipif(ref_lib.pose_lib() is None, reason="oracle/_ref/libpose_ref.so not built and no /root/reference to build it from")
 def test_oracle_pose_agrees_with_compiled_reference_g2o():
     cases = [dict(seed=s, frame=3 * s) for s in range(8)]
     cases += [dict(seed=s, frame=2 * s, n_planes=0, n_par=0, n_ver=0) for s in range(4)]                     # analytic Jacobians only
@@ -47,7 +45,6 @@ def test_oracle_pose_agrees_with_compiled_reference_g2o():
         _same(oracle_lib.pose_optimization(p), ref_lib.ref_pose_optimization(p))
 
 
-@pytest.mark.skipif(ref_lib.pose_lib() is None, reason="oracle/_ref/libpose_ref.so not built and no /root/reference to build it from")
 def test_oracle_translation_optimization_agrees_with_compiled_reference_g2o():
     """Optimizer::TranslationOptimization (src/Optimizer.cc:2995-3737) with the reference's OnlyTranslation edges: identical inlier counts and flags,
     rotation untouched on both sides, translation within 5e-6 m."""
@@ -64,7 +61,6 @@ def test_oracle_translation_optimization_agrees_with_compiled_reference_g2o():
         assert np.linalg.norm(o["Tcw_d"][:3, 3] - r["Tcw_d"][:3, 3]) < 5e-6, kw
 
 
-@pytest.mark.skipif(ref_lib.match_lib() is None, reason="oracle/_ref/libmatch_ref.so not built and no /root/reference to build it from")
 def test_oracle_pose_agrees_with_the_reference_functions_themselves():
     """Optimizer::PoseOptimization(Frame*) and Optimizer::TranslationOptimization(Frame*) called AS THEY ARE (src/Optimizer.cc compiled unmodified into
     libmatch_ref.so with Frame.cc / MapPoint.cc / MapLine.cpp / MapPlane.cc; oracle/ref/match_driver.cc only fills a Frame from the problem arrays and reads

@@ -3,8 +3,8 @@ Tracking + PoseOptimization, pose tolerance 1e-4 rad / 1e-3 m) against THE SAME 
 src/ORBextractor.cc (liborb_ref), Frame::ComputeStereoFromRGBD, ORBmatcher::SearchByProjection x2 with Frame::isInFrustum and the reference's
 feature grid, Optimizer::PoseOptimization(Frame*) (libmatch_ref: src/ORBmatcher.cc, Frame.cc, Optimizer.cc + Thirdparty/g2o compiled unmodified);
 only the glue between them (Tracking::TrackWithMotionModel / TrackLocalMap / the velocity update: pose products, the outlier sweep, the skip
-flags of SearchLocalPoints) is restated here in numpy with cv::Mat's float-storage / double-accumulation convention.  Falls back to the oracle
-restatements of the same functions when oracle/_ref is absent."""
+flags of SearchLocalPoints) is restated here in numpy with cv::Mat's float-storage / double-accumulation convention.  Where oracle/_ref is
+absent, the recorded answers of those functions stand in (ref_lib); the key points fed on are the oracle's, checked equal to the reference's."""
 import numpy as np
 import pytest
 
@@ -40,24 +40,24 @@ def _pose_problem(fa, matches, m, T0):
     return p, idx
 
 
-def _optimise(fa, matches, m, T, use_ref):
+def _optimise(fa, matches, m, T):
     p, idx = _pose_problem(fa, matches, m, T)
     if len(idx) < 3:
         return T, len(idx), 0
-    r = ref_lib.ref_full_pose_optimization(p, False) if use_ref else oracle_lib.pose_optimization(p)
+    r = ref_lib.ref_full_pose_optimization(p, False)
     matches[idx[r["outlier_pt"] != 0]] = -1
     return np.ascontiguousarray(r["Tcw"], np.float32), len(idx), int(r["n_inliers"])
 
 
 def _reference_chain(frames, m, T0):
-    use_ref = ref_lib.match_lib() is not None and ref_lib.orb_lib() is not None
-    s_last = oracle_lib.search_by_projection_last if not use_ref else ref_lib.ref_search_by_projection_last
-    s_map = oracle_lib.search_by_projection_map if not use_ref else ref_lib.ref_search_by_projection_map
+    s_last, s_map = ref_lib.ref_search_by_projection_last, ref_lib.ref_search_by_projection_map
     poses, stats = [], []
     T = np.ascontiguousarray(T0, np.float32)
     last = vel = fa_prev = matches_prev = None
     for t, (g, d) in enumerate(frames):
-        kps, desc = ref_lib.ref_orb_extract(g) if use_ref else oracle_lib.orb_extract(g)
+        kps, desc = oracle_lib.orb_extract(g)
+        rk, rd = ref_lib.ref_orb_extract(g)
+        assert ref_lib.same(rk, kps) and ref_lib.same(rd, desc), t
         fa = synth_map.frame_arrays(kps, desc, d)
         matches = np.full(fa["n"], -1, np.int32)
         st = [0, 0, 0, 0]
@@ -67,13 +67,13 @@ def _reference_chain(frames, m, T0):
             lf = dict(n=fa_prev["n"], keys=fa_prev["keys_un"], map_point=matches_prev, outlier=np.zeros(fa_prev["n"], np.uint8), Tcw=last)
             _, matches = s_last(synth_map.frame_view(fa, T), lf, m, 15.0, False, True, matches)
             matches = matches.copy()
-            T, st[0], st[1] = _optimise(fa, matches, m, T, use_ref)
+            T, st[0], st[1] = _optimise(fa, matches, m, T)
         mm = dict(m)
         mm["skip"] = m["skip"].copy()
         mm["skip"][matches[matches >= 0]] = 1
         _, matches, _ = s_map(synth_map.frame_view(fa, T), mm, 3.0, 0.8, matches)
         matches = matches.copy()
-        T, st[2], st[3] = _optimise(fa, matches, m, T, use_ref)
+        T, st[2], st[3] = _optimise(fa, matches, m, T)
         if t > 0:
             vel = _mm(T, _inv_pose(last))
         poses.append(T.copy()); stats.append(st)
